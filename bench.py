@@ -218,6 +218,20 @@ def reference_main(args):
 # ------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------
+def dump_outputs(dd, out_dir):
+    """What a caller of the timed path receives after its last step, as DIR/<name>.npy: the losses, the sampled
+    batch (indices, IS weights, TD errors, new priorities) and every parameter of the four networks."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"losses": np.array(dd.last_losses(), dtype=np.float32)}
+    for k, v in dd.last_batch_info().items():
+        out["batch_" + k] = v.cpu().numpy().astype(np.float64 if k == "idx" else np.float32)
+    for net in ("actor", "critic", "actor_target", "critic_target"):
+        for k, v in getattr(dd, net).state_dict().items():
+            out["%s.%s" % (net, k)] = v.cpu().numpy().astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def gpu_main(args):
     import torch
     import d4pg_b200 as d4pg
@@ -272,8 +286,8 @@ def gpu_main(args):
     sampler = ClockSampler(local)
     sampler.start()
     # the timed region = EXACTLY K steps between barrier + synchronize on both sides, CUDA events on the learner stream,
-    # max over ranks.  A region of K = 20 steps lasts ~2 ms, so it is measured R times back to back and the MEDIAN
-    # region is reported (every region is a complete, valid measurement; all of them are listed)
+    # max over ranks; --steps K is the number of timed steps.  A short region (K = 20 steps lasts ~2 ms) can be measured
+    # R = --repeats times back to back, and the MEDIAN region is reported (every region is listed)
     regions = []
     for _ in range(max(1, args.repeats)):
         barrier()
@@ -285,6 +299,8 @@ def gpu_main(args):
             e1.record(stream)
         barrier()
         regions.append(max_over_ranks(e0.elapsed_time(e1)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(dd, args.dump_outputs)
     ms = float(np.median(regions))
     kernels = dd.kernels_per_step()
     exchange = comm.exchange_mode() if comm is not None else "single"
@@ -442,7 +458,8 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=sorted(CFG))
     ap.add_argument("--no-cpu", action="store_true")
-    ap.add_argument("--repeats", type=int, default=5, help="timed regions of K steps each; the median region is reported")
+    ap.add_argument("--repeats", type=int, default=1, help="timed regions of K steps each; the median region is reported")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's outputs as DIR/<name>.npy")
     ap.add_argument("--precision", default="tf32x3", choices=["fp32", "tf32x3", "tf32"])
     ap.add_argument("--chain", type=int, default=1, help="MLP step plan: 1 = cluster-fused chains, 0 = one launch per level")
     args = ap.parse_args()

@@ -10,8 +10,6 @@ from /root/reference behind the 4-item compat shim in `oracle/ref_shim.py` and
 run in the build container:
   * `tests/golden/make_golden.py` dumps reference outputs to `tests/golden/*.npz`
     (NumPy 2.3.5 / torch 2.11.0 CPU dtype semantics, see SURVEY.md H11);
-  * `tests/test_oracle_vs_reference.py` re-checks the oracle against the live
-    reference whenever /root/reference exists (i.e. in the build container);
-  * `tests/test_oracle_golden.py` checks the oracle against the committed
-    fixtures everywhere (GPU box included).
+  * `tests/test_oracle_golden.py` and `tests/test_oracle_vs_reference.py` check
+    the oracle against the committed fixtures everywhere.
 """

@@ -10,19 +10,14 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    from oracle import ref_shim
-    have_ref = ref_shim.available()
     try:
         import torch
         have_gpu = torch.cuda.is_available()
     except Exception:
         have_gpu = False
     for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))

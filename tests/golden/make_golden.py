@@ -19,7 +19,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle import ref_shim  # noqa: E402
-from tests.helpers import ScriptedEnv  # noqa: E402
+from tests.helpers import NAMES, ScriptedEnv, digest, regen_init, transitions  # noqa: E402
 
 INFO51 = {"type": "categorical", "v_min": -50.0, "v_max": 0.0, "n_atoms": 51}
 INFO101 = {"type": "categorical", "v_min": -150.0, "v_max": 150.0, "n_atoms": 101}
@@ -352,6 +352,75 @@ def gen_baseline_sizes(ref):
     print("projection_c5_b4096.npz:", len(out), "arrays")
 
 
+def gen_oracle_vs_reference(ref):
+    """What tests/test_oracle_vs_reference.py compares the oracle with: reproject2 on random batches, reproject2 vs
+    reproj_categorical_dist at n_steps=5 (SURVEY H5), five DDPG.train() steps from a 650-transition PER buffer, and
+    the indices _sample_proportional draws from a pristine 2^16 tree.  Inputs the test can regenerate exactly (seeded
+    random.random() draws, the transitions) are pinned by their SHA-256; the softmax inputs are stored, since torch's
+    CPU softmax rounds differently with the vector width.  Outputs are stored whole where small, else as SHA-256."""
+    out = {}
+    rng = np.random.RandomState(5)
+    proj = {"probs": [], "r": [], "done": [], "m": []}
+    for trial in range(6):
+        B = 97
+        d = ref.ddpg.DDPG(3, 1, batch_size=B, critic_dist_info=INFO51, prioritized_replay=False, memory_size=4)
+        p = torch.softmax(torch.from_numpy(rng.randn(B, 51).astype(np.float32) * 3), 1).numpy()
+        r = (-60 * rng.rand(B)) if trial % 2 else -rng.randint(0, 3, B).astype(np.float64)
+        done = np.zeros(B, bool) if trial < 4 else (rng.rand(B) < 0.3)
+        if trial == 5:
+            r = -40 * rng.rand(B)      # terminal rows all non-integer, unclamped (no H6 mix)
+        for key, v in (("probs", p), ("r", r), ("done", done), ("m", digest(d.reproject2(p, r, done)))):
+            proj[key].append(v)
+    for key, v in proj.items():
+        out["proj_" + key] = np.stack(v)
+
+    rng = np.random.RandomState(6)
+    B = 32
+    d = ref.ddpg.DDPG(3, 1, batch_size=B, critic_dist_info=INFO51, prioritized_replay=False, memory_size=4, n_steps=5)
+    p = torch.softmax(torch.from_numpy(rng.randn(B, 51).astype(np.float32)), 1).numpy()
+    r = -3 * rng.rand(B)
+    done = np.zeros(B, bool)
+    out["h5_probs"], out["h5_r"], out["h5_done"] = p, r, done
+    out["h5_m_live"] = digest(d.reproject2(p, r, done))
+    out["h5_m_nstep"] = digest(d.reproj_categorical_dist(p.astype(np.float64), r, done.astype(np.float64)), np.float64)
+
+    B, mem, n_fill, steps, seed, data_seed = 48, 700, 650, 5, 21, 22
+    a0, c0 = regen_init(seed, 17, 6, 51)          # before make_learner_pair, which reseeds every generator
+    g, l, oa, oc = ref_shim.make_learner_pair(17, 6, INFO51, B, mem, seed=seed)
+    for k in NAMES:                 # the test rebuilds the initial weights from the seed
+        assert torch.equal(a0[k], l.actor.state_dict()[k]) and torch.equal(c0[k], l.critic.state_dict()[k]), k
+    rows = transitions(data_seed, n_fill, 17, 6)
+    for s, a, r, s2 in rows:
+        l.replayBuffer.add(s, a, r, s2, False)
+    out["train_meta"] = np.array([B, mem, n_fill, steps, seed, data_seed])
+    out["train_data"] = digest(np.concatenate([np.concatenate([s, a, [r], s2]) for s, a, r, s2 in rows]), np.float64)
+    us, tree, params = [], [], []
+    for t in range(steps):
+        random.seed(300 + t)
+        st = random.getstate()
+        us.append(digest(np.array([random.random() for _ in range(B)]), np.float64))
+        random.setstate(st)
+        l.train(g)
+        tree.append(digest(np.array([float(x) for x in l.replayBuffer._it_sum._value]), np.float64))
+        # [step, network (actor, critic, actor_target, critic_target), tensor (NAMES order)]
+        params.append([[digest(mod.state_dict()[k]) for k in NAMES]
+                       for mod in (l.actor, l.critic, l.actor_target, l.critic_target)])
+    out["train_u"], out["train_tree_sum"], out["train_params"] = np.stack(us), np.stack(tree), np.array(params)
+
+    size = 1 << 16
+    buf = ref.prioritized_replay_memory.PrioritizedReplayBuffer(size, alpha=0.6)
+    z = np.zeros(1, np.float32)
+    for i in range(size - 3):
+        buf.add(z, z, 0.0, z, False)
+    random.seed(5)
+    st = random.getstate()
+    out["pristine_u"] = digest(np.array([random.random() for _ in range(2000)]), np.float64)
+    random.setstate(st)
+    out["pristine_idx"] = np.array(buf._sample_proportional(2000), dtype=np.int32)
+    np.savez_compressed(os.path.join(HERE, "oracle_vs_reference.npz"), **out)
+    print("oracle_vs_reference.npz:", len(out), "arrays")
+
+
 def main():
     ref = ref_shim.load()
     torch.set_num_threads(1)
@@ -360,6 +429,9 @@ def main():
         return
     if len(sys.argv) > 1 and sys.argv[1] == "nstep":
         gen_nstep(ref)
+        return
+    if len(sys.argv) > 1 and sys.argv[1] == "oracle_vs_reference":
+        gen_oracle_vs_reference(ref)
         return
     gen_projection(ref)
     gen_tree(ref)
@@ -372,6 +444,7 @@ def main():
     gen_train(ref, "uniform_c1", 3, 1, INFO_PEND, 64, 500, 400, False, 3, 0.0, seed=13)
     gen_baseline_sizes(ref)
     gen_nstep(ref)
+    gen_oracle_vs_reference(ref)
 
 
 if __name__ == "__main__":

@@ -1,4 +1,5 @@
 """Shared test helpers: golden-fixture access and the compact-array comparison."""
+import hashlib
 import os
 
 import numpy as np
@@ -12,6 +13,13 @@ NAMES = ["fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias",
 
 def load(name):
     return np.load(os.path.join(GOLDEN, name))
+
+
+def digest(t, dtype=np.float32):
+    """SHA-256 of an array's values as `dtype`, as 32 uint8: bit-exact equality for arrays too large to store.  Adding
+    +0.0 maps -0.0 to +0.0, so two NaN-free arrays get the same digest exactly when np.array_equal holds for them."""
+    a = np.ascontiguousarray(torch.as_tensor(t).detach().cpu().numpy(), dtype=dtype) + dtype(0.0)
+    return np.frombuffer(hashlib.sha256(a.tobytes()).digest(), dtype=np.uint8)
 
 
 class ScriptedEnv(object):
@@ -61,6 +69,20 @@ def train_data(g):
     check_compact(g, "S", S, 0.0)
     check_compact(g, "R", R, 0.0)
     return S, A, R, S2, D
+
+
+def transitions(seed, n, obs_dim, act_dim):
+    """n (s, a, r, s2) rows drawn one at a time from RandomState(seed): f32 states and actions, f32-representable
+    Python-float rewards (what an environment loop hands to add())."""
+    rng = np.random.RandomState(seed)
+    rows = []
+    for _ in range(n):
+        s = rng.randn(obs_dim).astype(np.float32)
+        a = rng.uniform(-1, 1, act_dim).astype(np.float32)
+        r = float(np.float32(-3 * rng.rand()))
+        s2 = rng.randn(obs_dim).astype(np.float32)
+        rows.append((s, a, r, s2))
+    return rows
 
 
 def projection_c5_inputs():
