@@ -2,22 +2,10 @@
 #include "common.cuh"
 #include "gemm_ffma.cuh"
 #include <string.h>
-#include <stdlib.h>
 
 namespace d4pg {
 
 static thread_local char g_err[512] = "";
-
-int pdl_mode() {
-  static const int m = getenv("D4PG_PDL") ? atoi(getenv("D4PG_PDL")) : 0;
-  return m;
-}
-bool pdl_enabled() {
-  // measured on B200 (profiles/README.md): +17 % step time for the FFMA path, -5 % for the tcgen05 path
-  // -> opt-in.  D4PG_PDL=1 enables it.
-  static const bool on = getenv("D4PG_PDL") != nullptr;
-  return on;
-}
 
 void set_error(const char* fmt, ...) {
   va_list ap;

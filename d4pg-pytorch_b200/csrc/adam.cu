@@ -16,8 +16,6 @@ namespace d4pg {
 
 __global__ void __launch_bounds__(256) adam_polyak_kernel(const AdamArgs a) {
   __shared__ float red[2][8];
-  pdl_trigger(a.pdl);
-  pdl_wait();
   if (int(blockIdx.y) == a.nseg) {
     if (blockIdx.x == 0) adam_tail(a, red);
     return;
@@ -25,13 +23,11 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(const AdamArgs a) {
   step_stamp(a.trace, 7);
   adam_segment(a, blockIdx.y, blockIdx.x, gridDim.x);
   step_stamp(a.trace, 7 + 16);
-  pdl_trigger_end(a.pdl);
 }
 
 
 int launch_adam(const AdamArgs& a_in, cudaStream_t st) {
   AdamArgs a = a_in;
-  a.pdl = pdl_mode();
   a.trace = (a.clock && debug_trace_buffer()) ? debug_trace_buffer() + STEP_TRACE_BASE : nullptr;
   int64_t nmax = 0;
   for (int i = 0; i < a.nseg; ++i) nmax = a.seg[i].n > nmax ? a.seg[i].n : nmax;
@@ -40,7 +36,8 @@ int launch_adam(const AdamArgs& a_in, cudaStream_t st) {
   if (blocks < 1) blocks = 1;
   D4PG_MAX_CARVEOUT(adam_polyak_kernel);
   const int tail = ((a.clock || a.loss_out) && !a.skip_tail) ? 1 : 0;
-  D4PG_CUDA_OK(launch_pdl(adam_polyak_kernel, dim3(blocks, a.nseg + tail), dim3(256), 0, st, a));
+  adam_polyak_kernel<<<dim3(blocks, a.nseg + tail), 256, 0, st>>>(a);
+  D4PG_LAUNCH_OK();
   return D4PG_OK;
 }
 

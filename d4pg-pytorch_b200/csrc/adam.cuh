@@ -128,7 +128,6 @@ struct AdamArgs {
   int pipe_slot;                              // >= 0: the step's scalars are in this slot of the clock (prefetch pipeline)
   // fused tail (learner): deterministic batch means of the per-row losses -> out[0], out[1]
   const float* loss_rows; const float* pi_rows; int B; float inv_count; float* loss_out;
-  int pdl;                                    // programmatic-dependent-launch trigger position (0/1/2)
   int skip_tail;                              // 1: no loss means / clock advance in this launch (first of two Adam launches of a step)
 };
 int launch_adam(const AdamArgs& a, cudaStream_t st);

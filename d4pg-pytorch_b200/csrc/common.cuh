@@ -48,31 +48,10 @@ void set_error(const char* fmt, ...);
   } while (0)
 
 // ---- programmatic dependent launch (PDL) ---------------------------------------------------------
-// A step is ~18 small dependent kernels; at batch 256 the kernel boundaries (grid drain -> next grid
-// launch) cost as much as the kernels.  Every step kernel is launched with the programmatic-stream-
-// serialization attribute: it signals `launch_dependents` as soon as it starts, so the next kernel's
-// CTAs are scheduled (and run their prologue) while this one is still executing, and blocks in
-// `griddepcontrol.wait` until all of this kernel's memory is visible.  Captured into the CUDA graph
-// as programmatic dependency edges.  Opt-in with D4PG_PDL=1 (see pdl_enabled()).
-// PDL trigger position, carried in every step kernel's argument struct (`pdl` field):
-//   1 = `launch_dependents` at kernel entry (next grid becomes resident early), 2 = at kernel exit
+// Only the host pipeline's sample kernel is launched with the programmatic-stream-serialization attribute
+// (replay.cu: launch_sample): the tree add before it triggers early, the sample kernel waits for its writes.
 __device__ __forceinline__ void pdl_trigger_raw() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger(int mode) { if (mode == 1) pdl_trigger_raw(); }
-__device__ __forceinline__ void pdl_trigger_end(int mode) { if (mode == 2) pdl_trigger_raw(); }
-int pdl_mode();                      // 0 off, 1 early trigger, 2 late trigger (env D4PG_PDL)
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-bool pdl_enabled();
-template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                     Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
 
 // step timeline (D4PG_TC_TRACE): thread 0 of CTA 0 of every step kernel stamps %globaltimer at entry / exit
 __device__ __forceinline__ void step_stamp(unsigned long long* tr, int slot) {

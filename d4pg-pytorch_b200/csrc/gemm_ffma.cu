@@ -16,15 +16,12 @@ template <bool ALLOW_SPLIT>
 __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_ffma_kernel(const __grid_constant__ GemmBatch batch) {
   __shared__ __align__(16) float smem[2 * KC * LDS_A + 2 * KC * LDS_B];
   static_assert(2 * KC * LDS_A + 2 * KC * LDS_B >= GEMM_WARPS * BM * BN, "partial-tile buffer must fit");
-  pdl_trigger(batch.pdl);
-  pdl_wait();
   int pi = 0;
 #pragma unroll
   for (int i = 1; i < GEMM_MAX_PROBLEMS; ++i)
     if (i < batch.n && int(blockIdx.x) >= batch.p[i].tile_begin) pi = i;
   const GemmProblem P = batch.p[pi];        // one copy into registers (no constant-bank reads in the loops)
   gemm_tile_dispatch<ALLOW_SPLIT>(P, smem, blockIdx.x - P.tile_begin);
-  pdl_trigger_end(batch.pdl);
 }
 
 // Every dW of a step in one launch (mlp_chain.cuh: GemmWideBatch).  Only the asynchronous dW tile is
@@ -33,8 +30,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_ffma_kernel(const __grid
 template <bool ALLOW_SPLIT>
 __global__ void __launch_bounds__(GEMM_THREADS, 3) gemm_wide_kernel(const __grid_constant__ GemmWideBatch batch) {
   extern __shared__ __align__(16) float smem[];        // DW_SMEM_FLOATS
-  pdl_trigger(batch.pdl);
-  pdl_wait();
   int pi = 0;
 #pragma unroll
   for (int i = 1; i < GEMM_WIDE_MAX; ++i)
@@ -57,7 +52,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 3) gemm_wide_kernel(const __grid
     __syncthreads();
     if (threadIdx.x == 0) peer_signal_last_cta(batch.peer_sig, gridDim.x);
   }
-  pdl_trigger_end(batch.pdl);
 }
 
 // ---- host side -------------------------------------------------------------------------------
@@ -122,7 +116,7 @@ void gemm_batch_retile(GemmBatch& b, int bm, int bn) {
   }
 }
 void gemm_wide_begin(GemmWideBatch& b, const PeerSignal* sig) {
-  b.n = 0; b.total_tiles = 0; b.pdl = 0; b.trace = nullptr; b.has_peer_sig = sig ? 1 : 0;
+  b.n = 0; b.total_tiles = 0; b.trace = nullptr; b.has_peer_sig = sig ? 1 : 0;
   if (sig) b.peer_sig = *sig;
 }
 void gemm_wide_add(GemmWideBatch& b, const GemmProblem& pin) {
@@ -150,10 +144,10 @@ int gemm_wide_launch(GemmWideBatch& b, cudaStream_t st) {
     D4PG_CUDA_OK(cudaFuncSetAttribute(gemm_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     smem_set = true;
   }
-  b.pdl = pdl_mode();
   b.trace = debug_trace_buffer() ? debug_trace_buffer() + STEP_TRACE_BASE : nullptr;
-  if (split) D4PG_CUDA_OK(launch_pdl(gemm_wide_kernel<true>, dim3(b.total_tiles), dim3(GEMM_THREADS), smem, st, b));
-  else D4PG_CUDA_OK(launch_pdl(gemm_wide_kernel<false>, dim3(b.total_tiles), dim3(GEMM_THREADS), smem, st, b));
+  if (split) gemm_wide_kernel<true><<<b.total_tiles, GEMM_THREADS, smem, st>>>(b);
+  else gemm_wide_kernel<false><<<b.total_tiles, GEMM_THREADS, smem, st>>>(b);
+  D4PG_LAUNCH_OK();
   return D4PG_OK;
 }
 bool gemm_batch_has_splitk(const GemmBatch& b) {
@@ -172,9 +166,9 @@ int gemm_batch_launch(const GemmBatch& b, cudaStream_t st) {
                  "gemm_batch_launch: concat split K1=%d must be a multiple of %d", b.p[i].K1, KC);
   D4PG_MAX_CARVEOUT(gemm_ffma_kernel<false>);
   D4PG_MAX_CARVEOUT(gemm_ffma_kernel<true>);
-  const_cast<GemmBatch&>(b).pdl = pdl_mode();
-  if (gemm_batch_has_splitk(b)) D4PG_CUDA_OK(launch_pdl(gemm_ffma_kernel<true>, dim3(b.total_tiles), dim3(GEMM_THREADS), 0, st, b));
-  else D4PG_CUDA_OK(launch_pdl(gemm_ffma_kernel<false>, dim3(b.total_tiles), dim3(GEMM_THREADS), 0, st, b));
+  if (gemm_batch_has_splitk(b)) gemm_ffma_kernel<true><<<b.total_tiles, GEMM_THREADS, 0, st>>>(b);
+  else gemm_ffma_kernel<false><<<b.total_tiles, GEMM_THREADS, 0, st>>>(b);
+  D4PG_LAUNCH_OK();
   return D4PG_OK;
 }
 

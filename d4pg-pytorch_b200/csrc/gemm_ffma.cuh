@@ -41,7 +41,6 @@ struct GemmBatch {
   alignas(64) CUtensorMap tmap_a2[GEMM_MAX_PROBLEMS];   // concatenated tail of A (critic fc2's action columns)
   int all_tma;                                           // every operand of every problem is TMA-fed -> v2 kernel
   unsigned long long* trace;                             // optional %globaltimer phase stamps of CTA 0 (D4PG_TC_TRACE)
-  int pdl;                                               // programmatic-dependent-launch trigger position (0/1/2)
 };
 
 // host helpers ---------------------------------------------------------------------------

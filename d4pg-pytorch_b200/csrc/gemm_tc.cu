@@ -243,12 +243,10 @@ __global__ void __launch_bounds__(TC_THREADS) gemm_tc_kernel(const __grid_consta
     for (int i = 0; i < TC_NBARS; ++i) mbar_init(&bars[i], 1);
     mbar_fence_init();
   }
-  pdl_trigger(batch.pdl);
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
   const uint32_t tmem_d = tmem_base_s;
-  pdl_wait();                                   // prologue above overlapped the previous kernel's tail
 
   const CUtensorMap* tmA = &batch.tmap_a[pi];
   const CUtensorMap* tmB = &batch.tmap_b[pi];
@@ -289,7 +287,6 @@ __device__ __forceinline__ unsigned long long gtime() {
 
 __global__ void __launch_bounds__(T2_THREADS, 1) gemm_tc2_kernel(const __grid_constant__ GemmBatch batch, int passes) {
   extern __shared__ uint8_t smem_raw[];
-  pdl_trigger(batch.pdl);
   if (threadIdx.x == 0) TRACE(0);
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* lo_ring = smem + T2_STAGES * T2_STAGE;
@@ -325,8 +322,7 @@ __global__ void __launch_bounds__(T2_THREADS, 1) gemm_tc2_kernel(const __grid_co
   __syncthreads();
   tc_fence_after_sync();
   const uint32_t tmem_d = tmem_base_s;
-  pdl_wait();                                   // barrier init / TMEM alloc / descriptor prefetch overlapped the
-  if (threadIdx.x == 0) TRACE(1);               // previous kernel's tail; its results are visible from here on
+  if (threadIdx.x == 0) TRACE(1);
 
   if (warp == 0) {
     // ================================ TMA producer ==================================================
@@ -471,7 +467,6 @@ __global__ void __launch_bounds__(T2_THREADS, 1) gemm_tc2_kernel(const __grid_co
     }
   }
   if (tid == 64) TRACE(10);
-  pdl_trigger_end(batch.pdl);
   tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) tmem_dealloc(tmem_d, 64);
@@ -524,8 +519,6 @@ static bool tma_ok(const float* p, int ld) { return (reinterpret_cast<uintptr_t>
 
 // v2 eligibility: every operand of every problem can be described by a tensor map
 static bool prepare_v2(GemmBatch& b) {
-  static const bool disabled = getenv("D4PG_TC_V1") != nullptr;
-  if (disabled) return false;
   for (int i = 0; i < b.n; ++i) {
     const GemmProblem& p = b.p[i];
     if (!tma_ok(p.A, p.lda) || !tma_ok(p.Bm, p.ldb)) return false;
@@ -551,7 +544,6 @@ unsigned long long* debug_trace_buffer() {
   return tracing ? g_trace : nullptr;
 }
 void gemm_tc_prepare(GemmBatch& b) {
-  static const bool disabled = getenv("D4PG_NO_TMA") != nullptr;
   b.trace = debug_trace_buffer();
   b.all_tma = prepare_v2(b) ? 1 : 0;
   if (b.all_tma) { gemm_batch_retile(b, T2_BM, T2_BN); return; }
@@ -560,7 +552,6 @@ void gemm_tc_prepare(GemmBatch& b) {
   for (int i = 0; i < b.n; ++i) {
     GemmProblem& p = b.p[i];
     p.flags &= ~(GEMM_A_TMA | GEMM_B_TMA);
-    if (disabled) continue;
     if (p.mode != GEMM_DW && tma_ok(p.A, p.lda) && encode_kmajor(&b.tmap_a[i], p.A, p.K1, p.M, p.lda, TC_BM))
       p.flags |= GEMM_A_TMA;
     if (p.mode == GEMM_FWD && tma_ok(p.Bm, p.ldb) && encode_kmajor(&b.tmap_b[i], p.Bm, p.K, p.N, p.ldb, TC_BN))
@@ -581,9 +572,9 @@ int gemm_tc_batch_launch(const GemmBatch& b, int passes, cudaStream_t st) {
     D4PG_MAX_CARVEOUT(gemm_tc2_kernel);
     attr_set = true;
   }
-  const_cast<GemmBatch&>(b).pdl = pdl_mode();
-  if (b.all_tma) D4PG_CUDA_OK(launch_pdl(gemm_tc2_kernel, dim3(b.total_tiles), dim3(T2_THREADS), T2_SMEM, st, b, passes));
-  else D4PG_CUDA_OK(launch_pdl(gemm_tc_kernel, dim3(b.total_tiles), dim3(TC_THREADS), TC_SMEM, st, b, passes));
+  if (b.all_tma) gemm_tc2_kernel<<<b.total_tiles, T2_THREADS, T2_SMEM, st>>>(b, passes);
+  else gemm_tc_kernel<<<b.total_tiles, TC_THREADS, TC_SMEM, st>>>(b, passes);
+  D4PG_LAUNCH_OK();
   return D4PG_OK;
 }
 

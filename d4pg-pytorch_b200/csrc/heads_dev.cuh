@@ -252,8 +252,6 @@ __device__ __forceinline__ void heads_row(const HeadsArgs& a, int row, int lane,
 template <int MODE, int NT>
 __global__ void __launch_bounds__(HEAD_WARPS * 32) heads_kernel(const HeadsArgs a) {
   __shared__ HeadsWarpSmem ws[HEAD_WARPS];
-  pdl_trigger(a.pdl);
-  pdl_wait();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = blockIdx.x * HEAD_WARPS + warp;            // warps [0, B): critic part of row g; [B, 2B): policy head of row g - B
   step_stamp(a.trace, 2);
@@ -264,7 +262,6 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32) heads_kernel(const HeadsArgs 
   if (a.sampler_clock && blockIdx.x == 0 && threadIdx.x == 0) {
     a.sampler_clock->s_adam_step += 1; a.sampler_clock->s_beta_t += 1; a.sampler_clock->s_steps_done += 1;
   }
-  pdl_trigger_end(a.pdl);
 }
 
 }  // namespace d4pg

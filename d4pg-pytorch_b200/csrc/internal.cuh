@@ -20,7 +20,6 @@ struct HeadsArgs {
   // corrected-semantics switches (SURVEY.md section 8f.4; the reference does neither, H3 / H4):
   const float* is_weights;   // non-null: critic CE row i is scaled by the PER importance weight w_i
   int ce_priority;           // 1: priority = CE_i + eps instead of |sum_j m_ij q_ij| + eps
-  int pdl;                   // programmatic-dependent-launch trigger position (0/1/2)
   unsigned long long* trace;
   int only_policy;               // 1: only the policy head (pi_rows, dlogits_pi) -- the second loss launch of the post-update-critic plan
   LearnerClock* sampler_clock;   // prefetch pipeline: thread 0 advances the sampler's counters (after sample(k), before sample(k+1))

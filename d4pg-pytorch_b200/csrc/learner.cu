@@ -157,8 +157,7 @@ static bool tcc_shapes_ok(const d4pg_learner_config_t& c) {
 static int tcc_setup(d4pg_learner* L) {
   L->tcc_ok = false; L->tcc_images = nullptr;
   const d4pg_learner_config_t& c = L->cfg;
-  static const bool off = getenv("D4PG_NO_TCC") != nullptr;      // A/B switch: mma.sync chain tiles instead
-  if (!tcc_shapes_ok(c) || off) return D4PG_OK;
+  if (!tcc_shapes_ok(c)) return D4PG_OK;
   const d4pg_learner_buffers_t& b = L->buf;
   const NetDims& da = L->da; const NetDims& dc = L->dc;
   const int S = c.obs_dim, A = c.act_dim, N = c.n_atoms, H = D4PG_HIDDEN;
@@ -369,8 +368,7 @@ static int enqueue_step(d4pg_learner* L, cudaStream_t st, int par, bool cold, bo
   const bool h7 = (c.loss_flags & 4) != 0;
   D4PG_REQUIRE(!h7 || (tcc && c.world_size <= 1), D4PG_ENOTSUP, "post-update-critic actor gradient needs the tcgen05 chain plan (precision tf32x3 / tf32, chain plan, batch <= 512) on one GPU");
   const bool chain = plan == 1 && !tcc;
-  static const bool no_pre = getenv("D4PG_NO_PRE") != nullptr;          // A/B switch
-  const bool pre_ok = chain && c.precision == 0 && A <= 8 && !no_pre;   // pre-layers: fp32 tile, |a| <= 8
+  const bool pre_ok = chain && c.precision == 0 && A <= 8;             // pre-layers: fp32 tile, |a| <= 8
   if (tcc) {
     // 2''. the same three forward chains on the tensor cores (mlp_tc_chain.cu): clusters of 8 CTAs own 64 rows,
     // every layer a tcgen05.mma tile.  The hi/lo weight images are re-packed first (Adam / Polyak changed them).
@@ -511,12 +509,6 @@ static int enqueue_step(d4pg_learner* L, cudaStream_t st, int par, bool cold, bo
   if (c.prioritized || pf) {
     D4PG_CUDA_OK(cudaEventRecord(L->ev_fork, st));
     D4PG_CUDA_OK(cudaStreamWaitEvent(L->side, L->ev_fork, 0));
-    static const bool copy_first = getenv("D4PG_PIPE_COPY_FIRST") != nullptr;      // A/B switch
-    if (pf && copy_first) {
-      D4PG_CUDA_OK(cudaMemcpyAsync(b.idx, bidx, size_t(B) * sizeof(int32_t), cudaMemcpyDeviceToDevice, L->side));
-      if (b.weights && c.prioritized)
-        D4PG_CUDA_OK(cudaMemcpyAsync(b.weights, bwts, size_t(B) * sizeof(float), cudaMemcpyDeviceToDevice, L->side));
-    }
     // host pipeline: the write-back also opens the ingest gate of step k+1 (its tree add / presample wait for this step's
     // loss kernel -- which advanced the sampler clock -- and for the priorities)
     if (c.prioritized) RUN(launch_tree_update(L->replay, B, bidx, b.prio, L->side, host_pipe(c) ? L->gate_flag : nullptr));
@@ -530,7 +522,7 @@ static int enqueue_step(d4pg_learner* L, cudaStream_t st, int par, bool cold, bo
                          q ? o.s_b : o.s, q ? o.a_b : o.a, q ? o.r_b : o.r, q ? o.s2_b : o.s2, q ? o.done_b : o.done,
                          Sp, Ap, q, L->side));
     }
-    if (pf && !copy_first) {                           // the caller-visible copies of this step's indices / IS weights (off the
+    if (pf) {                                          // the caller-visible copies of this step's indices / IS weights (off the
       // path to the next batch: after the write-back and the prefetch)
       D4PG_CUDA_OK(cudaMemcpyAsync(b.idx, bidx, size_t(B) * sizeof(int32_t), cudaMemcpyDeviceToDevice, L->side));
       if (b.weights && c.prioritized)
@@ -919,8 +911,7 @@ static int launch_variant(d4pg_learner* L, cudaStream_t st, int par, bool cold) 
 }
 
 static bool inline_wait(const d4pg_learner* L) {
-  static const bool off = getenv("D4PG_PIPE_EVENT") != nullptr;      // A/B switch: stream event instead
-  return !off && step_plan(L->cfg) == 1 && L->cfg.precision >= 1 && L->tcc_ok && cdiv(L->cfg.batch, SAMPLE_ROWS) <= TCC_THREADS;
+  return step_plan(L->cfg) == 1 && L->cfg.precision >= 1 && L->tcc_ok && cdiv(L->cfg.batch, SAMPLE_ROWS) <= TCC_THREADS;
 }
 
 // host pipeline: sample + gather batch `par` from the device copy of this step's uniforms / positions (the launch the
@@ -933,7 +924,7 @@ static int presample(d4pg_learner* L, int par, const double* uniforms, const int
   return learner_sample(L->replay, c.batch, c.prioritized, uniforms, !c.prioritized ? positions : nullptr, c.philox_seed,
                         o.clock, cp, o.idx2[par], o.wts2[par], par ? o.s_b : o.s, par ? o.a_b : o.a, par ? o.r_b : o.r,
                         par ? o.s2_b : o.s2, par ? o.done_b : o.done, pitch4(c.obs_dim), pitch4(c.act_dim), par, st,
-                        getenv("D4PG_PIPE_NO_PDL") == nullptr, o.pipe_epoch);
+                        true, o.pipe_epoch);
 }
 
 // The host-facing step: stage this step's host inputs in pinned memory, H2D, the step, order the caller after it.

@@ -67,7 +67,7 @@ int launch_mlp_chain(ChainArgs& a, cudaStream_t st);
 constexpr int GEMM_WIDE_MAX = 12;
 struct GemmWideBatch {
   GemmProblem p[GEMM_WIDE_MAX];
-  int n, total_tiles, pdl;
+  int n, total_tiles;
   unsigned long long* trace;
   // data parallel over peer memory: the last CTA to finish publishes "this rank's gradient half is complete"
   // ([0] published step count, [1] local step count, [2] CTA ticket), see comm.cu

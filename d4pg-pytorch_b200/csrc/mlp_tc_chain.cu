@@ -87,9 +87,6 @@ __device__ __forceinline__ void tcc_wait(uint64_t* bar, uint32_t parity, unsigne
 #define TCC_CODE(kind, slot, rank) (unsigned(kind) | (unsigned(slot) << 8) | (unsigned(rank) << 16))
 enum { WD_LOADER_DFULL = 2, WD_MMA_WFULL = 3, WD_MMA_FULL = 4, WD_EPI_DFULL = 5 };
 
-// generic-proxy writes (shared AND global) -> ordered before later async-proxy (TMA / tensor core) accesses
-__device__ __forceinline__ void tcc_fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 // The MMA-issuing code runs WARP-UNIFORM (all 32 lanes execute the loop with identical values, so descriptors live in
 // uniform registers) and only the instruction is predicated on an elected lane: measured on B200 (tests/probe/
 // mma_probe2.cu) 25 cycles per 64x32x8 tcgen05.mma this way vs 50 from a single-lane branch and 150+ with per-thread
@@ -156,7 +153,7 @@ __device__ __forceinline__ bool tcc_group_active(const TccSlot& S, int g, int n0
 __device__ __forceinline__ bool tcc_slot_active(const TccSlot& S, int n0) { return tcc_group_active(S, 0, n0) || tcc_group_active(S, 1, n0); }
 
 // loader lane: the CTA's weight slices of one slot -> W buffer (one bulk copy per group)
-__device__ __forceinline__ void tcc_issue_weights(const TccSlot& S, int rank, int n0, uint8_t* Wb, uint64_t* wfull, int flags) {
+__device__ __forceinline__ void tcc_issue_weights(const TccSlot& S, int rank, int n0, uint8_t* Wb, uint64_t* wfull) {
   const uint32_t gbytes = uint32_t(S.nchunks) * TCC_W_CHUNK;
   uint32_t bytes = 0;
 #pragma unroll
@@ -165,12 +162,7 @@ __device__ __forceinline__ void tcc_issue_weights(const TccSlot& S, int rank, in
   mbar_expect_tx(wfull, bytes);
 #pragma unroll
   for (int g = 0; g < TCC_MAX_GROUPS; ++g)
-    if (tcc_group_active(S, g, n0)) {
-      if (flags & 1) {                           // debugging: one copy per chunk
-        for (int c = 0; c < S.nchunks; ++c)
-          tcc_bulk_load(Wb + g * gbytes + c * TCC_W_CHUNK, S.g[g].wimg + size_t(rank) * gbytes + size_t(c) * TCC_W_CHUNK, TCC_W_CHUNK, wfull);
-      } else tcc_bulk_load(Wb + g * gbytes, S.g[g].wimg + size_t(rank) * gbytes, gbytes, wfull);
-    }
+    if (tcc_group_active(S, g, n0)) tcc_bulk_load(Wb + g * gbytes, S.g[g].wimg + size_t(rank) * gbytes, gbytes, wfull);
 }
 
 __global__ void __cluster_dims__(TCC_CLUSTER, 1, 1) __launch_bounds__(TCC_THREADS, 1)
@@ -230,7 +222,7 @@ mlp_tc_chain_kernel(const __grid_constant__ TccArgs args) {
   // per-role state.  fph: bit b = parity of the NEXT completion of full[b] this thread will wait for (MMA issuer)
   uint32_t fph = 0;
   int nact = 0;                          // slots this CTA took part in so far: phase of wfull / dfull
-  if (warp == 0 && lane == 0 && tcc_slot_active(CH.slot[0], n0)) tcc_issue_weights(CH.slot[0], rank, n0, Wb, wfull, args.flags);
+  if (warp == 0 && lane == 0 && tcc_slot_active(CH.slot[0], n0)) tcc_issue_weights(CH.slot[0], rank, n0, Wb, wfull);
 
   for (int l = 0; l < ns; ++l) {
     const TccSlot& S = CH.slot[l];
@@ -246,7 +238,7 @@ mlp_tc_chain_kernel(const __grid_constant__ TccArgs args) {
         if (tr) tr[0] = tcc_gtime();
         if (active && S.nloads > 0) {
           // the cluster's generic-proxy stores to the planes (acquired by the barrier above) -> this thread's TMA reads
-          if (args.flags & 4) tcc_fence_proxy_async_all(); else asm volatile("fence.proxy.async.global;" ::: "memory");
+          asm volatile("fence.proxy.async.global;" ::: "memory");
           for (int i = 0; i < S.nloads; ++i) {
             const TccLoad L = S.ld[i];
             const uint32_t bytes = uint32_t(L.count) * TCC_A_CHUNK;
@@ -259,7 +251,7 @@ mlp_tc_chain_kernel(const __grid_constant__ TccArgs args) {
         // next slot's weights travel while this slot's epilogue and the barrier run
         if (l + 1 < ns && tcc_slot_active(CH.slot[l + 1], n0)) {
           if (active) tcc_wait(dfull, nact & 1, args.watchdog, TCC_CODE(WD_LOADER_DFULL, l, rank), nact);  // the weight buffer is free
-          tcc_issue_weights(CH.slot[l + 1], rank, n0, Wb, wfull, args.flags);
+          tcc_issue_weights(CH.slot[l + 1], rank, n0, Wb, wfull);
         }
       }
       __syncwarp();
@@ -634,10 +626,11 @@ int tcc_slot_group(TccArgs& a, int c, int slot, const TccImage& img, int epi, co
   return g.pub;
 }
 
+// A chunks per bulk copy: fewer, larger copies are faster, but above 2 the first MMA of a slot waits longer
+constexpr int TCC_LOAD_GROUP = 2;
 int launch_mlp_tc_chain(TccArgs& a, cudaStream_t st) {
   D4PG_REQUIRE(a.nchains > 0 && a.nchains <= TCC_MAX_CHAINS, D4PG_EINVAL, "launch_mlp_tc_chain: %d chains", a.nchains);
   D4PG_REQUIRE(a.passes == 1 || a.passes == 3, D4PG_EINVAL, "launch_mlp_tc_chain: passes %d", a.passes);
-  static const int gmax = [] { const char* e = getenv("D4PG_TCC_GROUP"); const int v = e ? atoi(e) : 2; return v < 1 ? 1 : (v > 8 ? 8 : v); }();
   for (int c = 0; c < a.nchains; ++c) {
     TccChain& ch = a.chain[c];
     bool x_clobbered = false;
@@ -654,7 +647,7 @@ int launch_mlp_tc_chain(TccArgs& a, cudaStream_t st) {
                    "launch_mlp_tc_chain: slot %d: %d groups x %d chunks exceed the weight buffer", l, s.ngroups, s.nchunks);
       // A buffers are direct-mapped: the j-th non-resident chunk of a slot lives in buffer j (0..7); a 9th one takes
       // buffer 8, the resident X chunk's, if this slot does not read X (and X is dead from then on).  Consecutive
-      // chunks of one plane in consecutive buffers travel as ONE bulk copy (at most `gmax` chunks each, so that the
+      // chunks of one plane in consecutive buffers travel as ONE bulk copy (at most TCC_LOAD_GROUP chunks each, so that the
       // MMAs of the first chunks overlap the arrival of the rest).
       int nring = 0;
       bool uses_x = false;
@@ -678,7 +671,7 @@ int launch_mlp_tc_chain(TccArgs& a, cudaStream_t st) {
         ++nring;
         if (k.kind == TCC_SRC_IMG) {
           TccLoad* cur = s.nloads ? &s.ld[s.nloads - 1] : nullptr;
-          if (cur && cur->plane == k.plane && cur->chunk0 + cur->count == k.chunk && cur->buf0 + cur->count == k.buf && cur->count < gmax) ++cur->count;
+          if (cur && cur->plane == k.plane && cur->chunk0 + cur->count == k.chunk && cur->buf0 + cur->count == k.buf && cur->count < TCC_LOAD_GROUP) ++cur->count;
           else s.ld[s.nloads++] = TccLoad{k.plane, k.chunk, k.buf, 1};
         }
       }
@@ -713,7 +706,6 @@ int launch_mlp_tc_chain(TccArgs& a, cudaStream_t st) {
     attr_set = true;
   }
   a.watchdog = tcc_watchdog_device();
-  { const char* e = getenv("D4PG_TCC_FLAGS"); a.flags = e ? atoi(e) : 0; }
   unsigned long long* dbg = debug_trace_buffer();
   a.trace = dbg ? dbg + (a.step_slot == 5 ? 384 : 256) : nullptr;
   a.step_trace = dbg ? dbg + STEP_TRACE_BASE : nullptr;

@@ -55,7 +55,6 @@ struct TccArgs {
   uint8_t* xchg;                  // [nchains][row_blocks][TCC_PLANES][TCC_PLANE_BYTES]
   unsigned long long* trace; int trace_cta;
   unsigned long long* step_trace; int step_slot;
-  int flags;                      // debugging switches (env D4PG_TCC_FLAGS)
   unsigned long long* watchdog;   // host-mapped record written by a wait that timed out (see tcc_wait)
 };
 

@@ -20,19 +20,19 @@ namespace d4pg {
 
 int launch_heads(const HeadsArgs& a_in, int mode, cudaStream_t st) {
   HeadsArgs a = a_in;
-  a.pdl = pdl_mode();
   a.trace = (a.sampler_clock && debug_trace_buffer()) ? debug_trace_buffer() + STEP_TRACE_BASE : nullptr;
   dim3 grid(cdiv(((a.pi_logits && !a.only_policy) ? 2 : 1) * a.B, HEAD_WARPS)), block(HEAD_WARPS * 32);   // policy heads on warps of their own
   D4PG_MAX_CARVEOUT((heads_kernel<0, 2>)); D4PG_MAX_CARVEOUT((heads_kernel<1, 2>));
   D4PG_MAX_CARVEOUT((heads_kernel<0, 4>)); D4PG_MAX_CARVEOUT((heads_kernel<1, 4>));
   // NT = atom slots per lane: 2 covers N<=64 (51 atoms), 4 covers N<=128 (101 atoms)
   if (a.N <= 64) {
-    if (mode == 0) D4PG_CUDA_OK(launch_pdl(heads_kernel<0, 2>, grid, block, 0, st, a));
-    else D4PG_CUDA_OK(launch_pdl(heads_kernel<1, 2>, grid, block, 0, st, a));
+    if (mode == 0) heads_kernel<0, 2><<<grid, block, 0, st>>>(a);
+    else heads_kernel<1, 2><<<grid, block, 0, st>>>(a);
   } else {
-    if (mode == 0) D4PG_CUDA_OK(launch_pdl(heads_kernel<0, 4>, grid, block, 0, st, a));
-    else D4PG_CUDA_OK(launch_pdl(heads_kernel<1, 4>, grid, block, 0, st, a));
+    if (mode == 0) heads_kernel<0, 4><<<grid, block, 0, st>>>(a);
+    else heads_kernel<1, 4><<<grid, block, 0, st>>>(a);
   }
+  D4PG_LAUNCH_OK();
   return D4PG_OK;
 }
 

@@ -12,7 +12,6 @@
 // Node dtype is fp32 -- what the reference's Python evaluates to under NumPy 2 (SURVEY.md H11).
 // Everything is HBM/L2 pointer chasing + row gathers: no tensor-core work here.
 #include "replay_dev.cuh"
-#include <stdlib.h>
 #include <new>
 #include <string.h>
 #include <algorithm>
@@ -44,7 +43,6 @@ static unsigned long long* step_trace() { unsigned long long* p = debug_trace_bu
 
 __global__ void __launch_bounds__(SAMPLE_THREADS) sample_gather_kernel(const SampleArgs a) {
   __shared__ SampleSmem sm;
-  pdl_trigger(a.pdl);
   pdl_wait();
   step_stamp(a.trace, a.trace_slot);
   sample_body(a, blockIdx.x, sm);
@@ -57,7 +55,6 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) sample_gather_kernel(const Sam
     }
   }
   step_stamp(a.trace, a.trace_slot + 16);
-  pdl_trigger_end(a.pdl);
 }
 
 template <int MODE>
@@ -287,23 +284,18 @@ int launch_sample(const d4pg_replay* h, SampleArgs& a, cudaStream_t st, bool dep
   a.sum = h->sum; a.mn = h->mn; a.cap = h->cap; a.state = reinterpret_cast<const ReplayState*>(h->state);
   a.obs = h->obs; a.act = h->act; a.rew = h->rew; a.obs2 = h->obs2; a.done = h->done;
   a.obs_dim = h->obs_dim; a.act_dim = h->act_dim;
-  a.pdl = pdl_mode();
   a.trace = (a.clock && debug_trace_buffer()) ? debug_trace_buffer() + STEP_TRACE_BASE : nullptr;
   a.trace_slot = a.pipe_slot >= 0 && a.uniforms == nullptr && st_is_side(st) ? 4 : 0;
   D4PG_MAX_CARVEOUT(sample_gather_kernel);
-  if (dependent) {
-    // programmatic dependent launch behind the previous kernel of the stream (the host pipeline's tree add): the grid is
-    // resident when that kernel ends, griddepcontrol.wait at the top of the kernel holds it until its writes are visible
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(cdiv(a.B, SAMPLE_ROWS)); cfg.blockDim = dim3(SAMPLE_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    D4PG_CUDA_OK(cudaLaunchKernelEx(&cfg, sample_gather_kernel, a));
-    return D4PG_OK;
-  }
-  D4PG_CUDA_OK(launch_pdl(sample_gather_kernel, dim3(cdiv(a.B, SAMPLE_ROWS)), dim3(SAMPLE_THREADS), 0, st, a));
+  // dependent: programmatic dependent launch behind the previous kernel of the stream (the host pipeline's tree add): the
+  // grid is resident when that kernel ends, pdl_wait() at the top of the kernel holds it until its writes are visible
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(cdiv(a.B, SAMPLE_ROWS)); cfg.blockDim = dim3(SAMPLE_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = dependent ? 1 : 0;
+  D4PG_CUDA_OK(cudaLaunchKernelEx(&cfg, sample_gather_kernel, a));
   return D4PG_OK;
 }
 
@@ -351,16 +343,14 @@ int launch_tree_update(d4pg_replay* h, int B, const int32_t* idx, const float* p
   a.sum = h->sum; a.mn = h->mn; a.cap = h->cap; a.log2cap = h->log2cap; a.size = h->size;
   a.n = B; a.idx = idx; a.v0 = prio; a.alpha_f32 = h->alpha_f32; a.scratch = h->scratch; a.state = reinterpret_cast<ReplayState*>(h->state);
   a.trace = (st_is_side(st) && debug_trace_buffer()) ? debug_trace_buffer() + STEP_TRACE_BASE : nullptr;
-  static const bool slow_tree = getenv("D4PG_TREE_SLOW") != nullptr;      // A/B switch for profiling
-  if (!slow_tree && B <= TREE_FAST_MAX && h->log2cap < TREE_FAST_LEVELS) {
+  if (B <= TREE_FAST_MAX && h->log2cap < TREE_FAST_LEVELS) {
     int hs = 64;
     while (hs < 2 * B) hs *= 2;
     const int threads = ((B + 31) / 32) * 32;
     const size_t smem = size_t(hs) * 2 * (sizeof(int) + sizeof(float2));     // 12 KB at B = 512
     D4PG_MAX_CARVEOUT(tree_update_fast_kernel);
     const int D = std::min(4, h->log2cap);                     // 2^D CTAs, one per top-level subtree
-    static const bool sig_kernel = getenv("D4PG_PIPE_SIGNAL_KERNEL") != nullptr;      // A/B switch: separate signal kernel
-    if (D > 0 && !sig_kernel) { a.gate = gate; gate = nullptr; }   // the last CTA opens the gate itself
+    if (D > 0) { a.gate = gate; gate = nullptr; }   // the last CTA opens the gate itself
     tree_update_fast_kernel<<<1 << D, threads, smem, st>>>(a, hs, D);
   } else {
     D4PG_MAX_CARVEOUT(tree_write_kernel<TREE_UPDATE>);
@@ -658,8 +648,7 @@ extern "C" int32_t d4pg_replay_add(d4pg_replay_t* h, int64_t n, const float* obs
     // the last launched learner step's priority write-back -- inside the first tree kernel when that is the 1-CTA fast one
     const int64_t n1g = std::min<int64_t>(n, h->size - start);
     const unsigned long long* gflag = nullptr; unsigned long long gtarget = 0;
-    static const bool gate_kernel = getenv("D4PG_PIPE_GATE_KERNEL") != nullptr;      // A/B switch: separate 1-thread gate kernel
-    if (h->gate_pending && !gate_kernel && n <= 65536 && n1g <= TREE_ADD_FAST_MAX && h->log2cap < 32) {
+    if (h->gate_pending && n <= 65536 && n1g <= TREE_ADD_FAST_MAX && h->log2cap < 32) {
       gflag = h->gate_flag; gtarget = h->gate_target; h->gate_pending = false;
     } else {
       int grc = replay_gate_consume(h, st); if (grc) return grc;

@@ -68,7 +68,6 @@ struct SampleArgs {
   int uniform_mode;                 // 1: idx = floor(u*len) (device-side uniform replay, with replacement)
   int32_t* idx; float* weights;
   float* s; float* a; double* r; float* s2; uint8_t* d;
-  int pdl;                          // programmatic-dependent-launch trigger position (0/1/2)
   int pipe_slot;                    // >= 0 (prefetch pipeline): use the sampler's own counters, derive into this slot
   unsigned long long* trace; int trace_slot;
   unsigned long long* done_epoch;   // host pipeline: CTA b publishes (release) s_steps_done + 1 in [b] when its rows are gathered

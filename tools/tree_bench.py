@@ -1,5 +1,5 @@
 """python tools/tree_bench.py : device time of one update_priorities call (256 leaves, capacity 2^20), CUDA events,
-with an L2 flush between calls.  D4PG_TREE_SLOW=1 selects the level-synchronous kernel."""
+with an L2 flush between calls.  At this size the update runs the fast multi-CTA kernel (tree_update_fast_kernel)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
